@@ -2,7 +2,7 @@
 """bench.py — Groth16 prove throughput on B200 (the driver's contract).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload prove|g1msm|g2msm|verify]
-                    [--logn L] [--with-qap]
+                    [--logn L] [--with-qap] [--dump-outputs DIR]
 
 Default workload (BASELINE.json's metric): one step = one groth16.GenerateProofs (groth16/groth16.go:225-278) on the
 synthetic R1CS shape of SURVEY §8(d): n = 2^20 constraints, m = n+2 signals, NPublic = 1, full-width witness.
@@ -24,6 +24,12 @@ Other workloads (BASELINE.json configs 3 and 5; never the default line):
 `--impl reference` times the reference's own algorithm (oracle/ref_c.c: per-term MSB-first double-and-add + add-2007-bl
 accumulate, exactly groth16.go:243-271) on the host cores, on a fixed-size sample of the same workload; nothing of the
 GPU library is loaded in that arm.
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy in float64: prove -> PiA, PiB, PiC;
+g1msm / g2msm -> msm; verify -> pairing (a seeded sample of at most 4096 results of the batch) and pairing_rows (their
+indices).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.  Every
+F_q value is stored as its eight little-endian 32-bit words (exact in float64).  Curve points are stored in affine form
+(x, y): the Jacobian representative the library returns depends on the order of additions inside a bucket.
 """
 import argparse
 import ctypes
@@ -66,7 +72,32 @@ def parse():
                          "latency chains of one proof overlap the accumulation of the other; 1 = one proof at a time)")
     ap.add_argument("--pairing-kernel", type=int, default=None, choices=[0, 1, 2], help="A/B (verify workload): b200_pairing_batch with one thread (1) / one warp (2) per pairing")
     ap.add_argument("--tma-staging", type=int, default=None, choices=[0, 1, 2], help="A/B: staged backward pass off / all rounds / rounds >= 2")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float64, see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def _fq_words(vals):
+    """F_q values -> their eight little-endian 32-bit words each."""
+    from gosnark_b200._lib import ints_to_limbs
+    return ints_to_limbs(vals).view(np.uint32)
+
+
+def affine_words(group, p):
+    """A Jacobian point of the oracle's G1 / G2 -> its affine x, y as 32-bit words: shape (2, 8) for G1, (2, 2, 8) for G2."""
+    x, y = group.affine(p)[:2]
+    if isinstance(x, tuple):
+        return _fq_words([*x, *y]).reshape(2, 2, 8)
+    return _fq_words([x, y]).reshape(2, 8)
+
+
+def dump_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # --------------------------------------------------------------------------- clocks
@@ -267,7 +298,7 @@ def run_reference(args):
     ref = CpuReference()
     for _ in range(args.warmup):
         ref.per_term()
-    v, info = reference_value(ref, args.workload, n, max(args.steps, 5))
+    v, info = reference_value(ref, args.workload, n, args.steps)
     if args.workload != "prove":
         v = v * n / 1e6                      # MSMs per second -> Mscalar-mul/s
     info["value"], info["unit"] = v, unit
@@ -512,6 +543,7 @@ def run_prove(args, c):
     prof0 = (ctypes.c_double * 8)()
     check(L.b200_profile_read(prof0))          # reset counters
     ms_total = timed(c, step_in_flight, args.steps, profile=args.profile_region, extra_streams=fly_streams[1:])
+    last_out = d_outs[(fly_ctr[0] - 1) % n_fly].cpu().numpy().view(np.uint64) if args.dump_outputs and rank == 0 else None
     prof = (ctypes.c_double * 8)()
     check(L.b200_profile_read(prof))
     check(L.b200_profile(0))
@@ -529,7 +561,7 @@ def run_prove(args, c):
         step_device()
     torch.cuda.synchronize()
     check(L.b200_profile_read(prof0))
-    ser_steps = max(2, args.steps // 2)
+    ser_steps = args.steps
     ms_serial = timed(c, step_device, ser_steps) / ser_steps
     prof_x = (ctypes.c_double * 8)()
     check(L.b200_profile_read(prof_x))
@@ -647,7 +679,7 @@ def run_prove(args, c):
         line["verified_under_real_vk"] = verified
     if not args.no_extras and world == 1 and not args.with_qap:
         try:
-            line["g1_msm_2p20"] = side_g1_msm(c)
+            line["g1_msm_2p20"] = side_g1_msm(c, steps=args.steps, warmup=args.warmup)
         except Exception as e:   # a side measurement must never take the bench line down
             line["g1_msm_2p20"] = {"error": str(e)}
     if not args.no_extras and world == 1:
@@ -659,11 +691,15 @@ def run_prove(args, c):
             line["cpu_baseline"] = cinfo
         except Exception as e:   # the checker must never take the bench line down
             line["cpu_baseline"] = {"error": str(e)}
+    if last_out is not None:
+        pa, pc = _unflatten_g1(last_out[:24])
+        dump_outputs(args.dump_outputs, {"PiA": affine_words(G1o, pa), "PiB": affine_words(G2o, _unflatten_g2(last_out[24:])[0]),
+                                         "PiC": affine_words(G1o, pc)})
     print(json.dumps(line))
     return 0
 
 
-def side_g1_msm(c, logn=20, steps=10, warmup=3):
+def side_g1_msm(c, steps, warmup, logn=20):
     """The other half of BASELINE.json's metric inside the default line: a stand-alone BN128 G1 MSM of 2^logn random scalars /
     points (config 3), device-resident — two MSMs in flight on two base-set objects, and one at a time."""
     torch, L = c.torch, c.L
@@ -802,6 +838,12 @@ def run_msm(args, c):
     torch.cuda.synchronize()
     ms = timed(c, step_in_flight, args.steps, profile=args.profile_region, extra_streams=fly_streams[1:]) / args.steps
     clk = clocks.stop() if rank == 0 else None
+    last_msm = None
+    if args.dump_outputs:
+        k_last = (fly_ctr[0] - 1) % n_fly
+        last_msm = np.zeros(words, dtype=np.uint64)
+        check((L.b200_g1_sum_partials if group == 1 else L.b200_g2_sum_partials)(
+            (d_alls[k_last] if world > 1 else d_parts[k_last]).data_ptr(), world, ptr(last_msm), st))
     # one MSM at a time (its latency), with CUDA events around its accumulation phase for the roofline
     check(L.b200_profile(1))
     prof = (ctypes.c_double * 8)()
@@ -852,6 +894,8 @@ def run_msm(args, c):
             line["cpu_baseline"] = cinfo
         except Exception as e:
             line["cpu_baseline"] = {"error": str(e)}
+    if last_msm is not None:
+        dump_outputs(args.dump_outputs, {"msm": affine_words(G, (_unflatten_g1(last_msm) if group == 1 else _unflatten_g2(last_msm))[0])})
     print(json.dumps(line))
     return 0
 
@@ -915,6 +959,9 @@ def run_verify(args, c):
     for _ in range(reps):
         ok = ok and syn.verify(pa, pb, pc)
     verify_ms = (time.perf_counter() - t0) * 1e3 / reps
+    if args.dump_outputs:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, 4096), replace=False))
+        dump_outputs(args.dump_outputs, {"pairing": out[rows].view(np.uint32).reshape(len(rows), 12, 8), "pairing_rows": rows})
     metric, unit = metric_of("verify")
     print(json.dumps({"metric": metric, "value": n / ms * 1e3, "unit": unit, "n_gpus": 1, "steps": args.steps, "warmup": args.warmup,
                       "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u256 (mod q), F_q^12",

@@ -4,21 +4,19 @@ UNMODIFIED Go binary's verify commands accept it."""
 import json
 import os
 import shutil
-import subprocess
 import tempfile
 
 import pytest
 
+import gocli
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GOBIN = os.path.join(ROOT, "oracle", "_ref", "go-snark-cli")
 
 
 @pytest.mark.parametrize("name,proto", [("x3x5", "groth16"), ("chain21", "groth16"), ("x3x5", "pinocchio")])
-def test_go_cli_verifies_files_we_write(golden_dir, name, proto):
-    if not os.path.exists(GOBIN):
-        pytest.skip("oracle/_ref/go-snark-cli not staged")
+def test_go_cli_verifies_files_we_write(golden_dir, name, proto, monkeypatch):
     from gosnark_b200 import cli
+    gocli.seed_rand_fr(monkeypatch, 1)
     g = json.load(open(os.path.join(golden_dir, f"gobin_{name}.json")))
     d = tempfile.mkdtemp(prefix="clif_")
     cwd = os.getcwd()
@@ -31,12 +29,7 @@ def test_go_cli_verifies_files_we_write(golden_dir, name, proto):
         os.chdir(d)
         assert cli.main(["groth16", "genproofs"] if proto == "groth16" else ["genproofs"]) == 0
         os.chdir(cwd)
-        b = os.path.join(d, "gsc")
-        shutil.copy(GOBIN, b)
-        os.chmod(b, 0o755)
-        p = subprocess.run([b, *(["groth16", "verify"] if proto == "groth16" else ["verify"])], cwd=d,
-                           capture_output=True, text=True, timeout=120)
-        out = p.stdout + p.stderr
+        out = gocli.run(d, *(["groth16", "verify"] if proto == "groth16" else ["verify"]))
         assert ("verification passed" in out) if proto == "groth16" else ("Proofs verified" in out and "❌" not in out), out
     finally:
         os.chdir(cwd)

@@ -3,17 +3,15 @@ tests/test_snark_host_logic.py and tests/test_utils_parsers.py exercise on the C
 import json
 import os
 import shutil
-import subprocess
 import tempfile
 
 import pytest
 
+import gocli
 from oracle import ref_py as o
 from test_utils_parsers import K5, K5_PIB
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GOBIN = os.path.join(ROOT, "oracle", "_ref", "go-snark-cli")
 G1, G2 = o.BN.G1, o.BN.G2
 
 
@@ -54,12 +52,11 @@ def test_verify_from_circom_files(golden_dir, tmp_path):
 
 
 @pytest.mark.parametrize("proto", ["groth16", "pinocchio"])
-def test_cli_trustedsetup_prove_verify_with_go_in_the_loop(golden_dir, proto, capsys):
+def test_cli_trustedsetup_prove_verify_with_go_in_the_loop(golden_dir, proto, capsys, monkeypatch):
     """Our `trustedsetup` (GPU-minted CRS) -> Go `genproofs` + `verify` accept it -> our `genproofs` overwrites
     proofs.json -> Go `verify` and our `verify` accept that too (cli/main.go:231-549)."""
-    if not os.path.exists(GOBIN):
-        pytest.skip("oracle/_ref/go-snark-cli not staged")
     from gosnark_b200 import cli
+    gocli.seed_rand_fr(monkeypatch, 2)
     g = json.load(open(os.path.join(golden_dir, "gobin_x3x5.json")))
     d = tempfile.mkdtemp(prefix="clizz_")
     cwd = os.getcwd()
@@ -72,20 +69,16 @@ def test_cli_trustedsetup_prove_verify_with_go_in_the_loop(golden_dir, proto, ca
             json.dump(g[key], open(os.path.join(d, fname), "w"))
         os.chdir(d)
         assert cli.main(pre + ["trustedsetup"]) == 0
-        b = os.path.join(d, "gsc")
-        shutil.copy(GOBIN, b)
-        os.chmod(b, 0o755)
-        run = lambda *a: subprocess.run([b, *pre, *a], cwd=d, capture_output=True, text=True, timeout=120)
-        p = run("genproofs")
-        assert os.path.exists("proofs.json"), p.stdout[-400:] + p.stderr[-400:]
-        p = run("verify")
-        assert ok_text(p.stdout + p.stderr), p.stdout + p.stderr
+        out = gocli.run(d, *pre, "genproofs")
+        assert os.path.exists("proofs.json"), out[-800:]
+        out = gocli.run(d, *pre, "verify")
+        assert ok_text(out), out
         capsys.readouterr()
         assert cli.main(pre + ["verify"]) == 0                       # Go's proof, our verifier
         assert "Proofs verified" in capsys.readouterr().out
         assert cli.main(pre + ["genproofs"]) == 0                    # our proof under our setup
-        p = run("verify")
-        assert ok_text(p.stdout + p.stderr), p.stdout + p.stderr
+        out = gocli.run(d, *pre, "verify")
+        assert ok_text(out), out
         capsys.readouterr()
         assert cli.main(pre + ["verify"]) == 0
         assert "Proofs verified" in capsys.readouterr().out

@@ -1,21 +1,20 @@
 """GPU parity tests for the prove paths through the C ABI:
   snark.GenerateProofs   (snark.go:254-289)  — bit-exact (affine) vs the Go binary's proofs.json
   groth16.GenerateProofs (groth16.go:225-278) — vs the oracle with injected r,s, verified by the
-                                               oracle's VerifyProof and (when staged) by real Go code
+                                               oracle's VerifyProof and by real Go code (tests/gocli.py)
 """
 import json
 import os
 import random
 import shutil
-import subprocess
 import tempfile
 
 import pytest
 
+import gocli
 from oracle import ref_py as o
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G1, G2 = o.BN.G1, o.BN.G2
 
 
@@ -84,21 +83,14 @@ def test_pinocchio_matches_go_binary(mods, golden_dir, name):
 
 def go_verify(g, proof_json, cmd):
     """Have the reference's real Go code verify our proof (cli/main.go verify commands)."""
-    binary = os.path.join(ROOT, "oracle", "_ref", "go-snark-cli")
-    if not os.path.exists(binary):
-        return None
     d = tempfile.mkdtemp(prefix="gsv_")
     try:
-        b = os.path.join(d, "gsc")
-        shutil.copy(binary, b)
-        os.chmod(b, 0o755)
         key = "groth16_setup" if cmd[0] == "groth16" else "pinocchio_setup"
         for fname, obj in (("trustedsetup.json", g[key]), ("compiledcircuit.json", g["compiledcircuit"]),
                            ("publicInputs.json", g["public"]), ("proofs.json", proof_json)):
             with open(os.path.join(d, fname), "w") as f:
                 json.dump(obj, f)
-        p = subprocess.run([b, *cmd], cwd=d, capture_output=True, text=True, timeout=120)
-        return p.stdout + p.stderr
+        return gocli.run(d, *cmd)
     finally:
         shutil.rmtree(d)
 
@@ -123,8 +115,7 @@ def test_groth16_vs_oracle_and_verifiers(mods, golden_dir, name):
         assert not o.groth16_verify(vk, proof, [g["public"][0] - 1])
     out = go_verify(g, {"PiA": list(proof["PiA"]), "PiB": [list(c) for c in proof["PiB"]], "PiC": list(proof["PiC"])},
                     ["groth16", "verify"])
-    if out is not None:
-        assert "verification passed" in out, out
+    assert "verification passed" in out, out
     # fresh randomness path (like the reference): still a valid proof, different every time
     p1 = groth16.GenerateProofs(cc, pk, g["witness"], g["px"])
     p2 = groth16.GenerateProofs(cc, pk, g["witness"], g["px"])
@@ -137,8 +128,6 @@ def test_pinocchio_go_binary_verifies_our_proof(mods, golden_dir):
     proof = snark.GenerateProofs(g["compiledcircuit"], pinocchio_pk(g["pinocchio_setup"]), g["witness"], g["px"])
     pj = {k: (list(v) if k != "PiB" else [list(c) for c in v]) for k, v in proof.items()}
     out = go_verify(g, pj, ["verify"])
-    if out is None:
-        pytest.skip("oracle/_ref/go-snark-cli not staged")
     assert "Proofs verified" in out and "❌" not in out, out
 
 

@@ -5,16 +5,15 @@ import json
 import os
 import random
 import shutil
-import subprocess
 import tempfile
 
 import numpy as np
 import pytest
 
+import gocli
 from oracle import ref_py as o
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 R = o.R
 
 
@@ -141,21 +140,14 @@ def test_r1cs_load_argument_errors(mods):
 
 
 def go_groth16_verify(vk_json, proof_json, public):
-    binary = os.path.join(ROOT, "oracle", "_ref", "go-snark-cli")
-    if not os.path.exists(binary):
-        return None
     d = tempfile.mkdtemp(prefix="gsv_")
     try:
-        b = os.path.join(d, "gsc")
-        shutil.copy(binary, b)
-        os.chmod(b, 0o755)
         # the prebuilt binary also opens compiledcircuit.json (unused by VerifyProof): an empty object will do
         for fname, obj in (("trustedsetup.json", {"Vk": vk_json}), ("publicInputs.json", public), ("proofs.json", proof_json),
                            ("compiledcircuit.json", {})):
             with open(os.path.join(d, fname), "w") as f:
                 json.dump(obj, f)
-        p = subprocess.run([b, "groth16", "verify"], cwd=d, capture_output=True, text=True, timeout=300)
-        return p.stdout + p.stderr
+        return gocli.run(d, "groth16", "verify")
     finally:
         shutil.rmtree(d)
 
@@ -204,7 +196,6 @@ def test_real_crs_witness_to_verified_proof(mods, logn):
                "G2": {k: [list(cc) for cc in _unflatten_g2(v)[0]] for k, v in
                       (("Beta", syn.beta2), ("Gamma", syn.gamma2), ("Delta", syn.delta2))}}
     out = go_groth16_verify(vk_json, {"PiA": list(A), "PiB": [list(cc) for cc in B], "PiC": list(C)}, syn.circuit.public_signals)
-    if out is not None:
-        assert "Proofs verified" in out and "not verified" not in out, out
+    assert "Proofs verified" in out and "not verified" not in out, out
     check(lib().b200_pk_free(pk))
     syn.r1cs.free()

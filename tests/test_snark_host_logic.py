@@ -5,17 +5,15 @@ behaviour.  The kernels underneath are covered by the -m gpu tests of the same m
 import json
 import os
 import shutil
-import subprocess
 import tempfile
 
 import pytest
 
 import abi_standin
+import gocli
 from oracle import ref_py as o
 
 pytestmark = pytest.mark.slow
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GOBIN = os.path.join(ROOT, "oracle", "_ref", "go-snark-cli")
 TOX = {"T": 0x1234567, "Ka": 0x1111, "Kb": 0x2222, "Kc": 0x3333, "Kbeta": 0x4444, "Kgamma": 0x5555, "RhoA": 0x6666,
        "RhoB": 0x7777}
 
@@ -49,24 +47,20 @@ def test_pinocchio_setup_equals_oracle_and_go_accepts_it(flow):
     proof, _ = o.pinocchio_prove(cc["NVars"], cc["NPublic"], setup["Pk"], w, px)
     assert snark.VerifyProof(setup["Vk"], proof, [35])
     assert not snark.VerifyProof(setup["Vk"], proof, [34])
-    if os.path.exists(GOBIN):                                    # the reference's own verifier on the minted setup
-        d = tempfile.mkdtemp(prefix="pin_")
-        try:
-            pk = setup["Pk"]
-            js = {"Toxic": {k: None for k in setup["Toxic"]}, "G1T": [_lists(p) for p in pk["G1T"]], "G2T": None,
-                  "Pk": {k: ([_lists(p) for p in v] if k != "Z" else v) for k, v in pk.items() if k != "G1T"},
-                  "Vk": {k: ([_lists(p) for p in v] if k == "IC" else _lists(v)) for k, v in setup["Vk"].items()}}
-            for name, obj in (("trustedsetup.json", js), ("proofs.json", {k: _lists(v) for k, v in proof.items()}),
-                              ("compiledcircuit.json", cc), ("publicInputs.json", g["public"]),
-                              ("privateInputs.json", g["private"])):
-                json.dump(obj, open(os.path.join(d, name), "w"))
-            b = os.path.join(d, "gsc")
-            shutil.copy(GOBIN, b)
-            os.chmod(b, 0o755)
-            out = subprocess.run([b, "verify"], cwd=d, capture_output=True, text=True, timeout=120).stdout
-            assert "Proofs verified" in out and "❌" not in out, out
-        finally:
-            shutil.rmtree(d)
+    d = tempfile.mkdtemp(prefix="pin_")                          # the reference's own verifier on the minted setup
+    try:
+        pk = setup["Pk"]
+        js = {"Toxic": {k: None for k in setup["Toxic"]}, "G1T": [_lists(p) for p in pk["G1T"]], "G2T": None,
+              "Pk": {k: ([_lists(p) for p in v] if k != "Z" else v) for k, v in pk.items() if k != "G1T"},
+              "Vk": {k: ([_lists(p) for p in v] if k == "IC" else _lists(v)) for k, v in setup["Vk"].items()}}
+        for name, obj in (("trustedsetup.json", js), ("proofs.json", {k: _lists(v) for k, v in proof.items()}),
+                          ("compiledcircuit.json", cc), ("publicInputs.json", g["public"]),
+                          ("privateInputs.json", g["private"])):
+            json.dump(obj, open(os.path.join(d, name), "w"))
+        out = gocli.run(d, "verify")
+        assert "Proofs verified" in out and "❌" not in out, out
+    finally:
+        shutil.rmtree(d)
 
 
 def test_pinocchio_verify_go_proof_check_order_and_messages(flow, capsys):
@@ -134,10 +128,9 @@ def test_verify_from_circom_files(monkeypatch, golden_dir, tmp_path, capsys):
 def test_cli_trustedsetup_files_feed_the_go_binary(monkeypatch, golden_dir, proto, capsys):
     """File-level interop in the other direction (cli/main.go:231-301, 407-453): OUR `trustedsetup` writes
     trustedsetup.json, the UNMODIFIED Go binary proves with it and verifies; our `verify` accepts the Go proof."""
-    if not os.path.exists(GOBIN):
-        pytest.skip("oracle/_ref/go-snark-cli not staged")
     abi_standin.install(monkeypatch)
     from gosnark_b200 import cli
+    gocli.seed_rand_fr(monkeypatch, 3)
     g = json.load(open(os.path.join(golden_dir, "gobin_x3x5.json")))
     d = tempfile.mkdtemp(prefix="clits_")
     cwd = os.getcwd()
@@ -150,13 +143,9 @@ def test_cli_trustedsetup_files_feed_the_go_binary(monkeypatch, golden_dir, prot
         assert cli.main(pre + ["trustedsetup"] + (["wasm"] if proto == "pinocchio" else [])) == 0
         written = json.load(open("trustedsetup.json"))
         assert all(v is None for v in written["Toxic"].values())          # toxic waste is not written (main.go:273-277)
-        b = os.path.join(d, "gsc")
-        shutil.copy(GOBIN, b)
-        os.chmod(b, 0o755)
-        p = subprocess.run([b, *pre, "genproofs"], cwd=d, capture_output=True, text=True, timeout=120)
-        assert os.path.exists("proofs.json"), p.stdout[-500:] + p.stderr[-500:]
-        p = subprocess.run([b, *pre, "verify"], cwd=d, capture_output=True, text=True, timeout=120)
-        out = p.stdout + p.stderr
+        out = gocli.run(d, *pre, "genproofs")
+        assert os.path.exists("proofs.json"), out[-1000:]
+        out = gocli.run(d, *pre, "verify")
         assert ("verification passed" in out) if proto == "groth16" else ("Proofs verified" in out and "❌" not in out), out
         capsys.readouterr()
         assert cli.main(pre + ["verify"]) == 0
