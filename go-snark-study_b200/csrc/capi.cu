@@ -26,6 +26,7 @@
 #ifndef B200_NO_PAIRING
 #include "pairing.cuh"
 #include "pairing_warp.cuh"
+#include "verify_batch.cuh"
 #endif
 
 using namespace b200;
@@ -860,15 +861,14 @@ __global__ void __launch_bounds__(32 * kPairWarps) k_pairing_batch_warp(const Fq
   }
 }
 // groth16.VerifyProof (groth16/groth16.go:281-305): e(A,B) == e(alpha,beta) * (e(icPubl,gamma) * e(C,delta)).
-// pts1: A, alpha1, icPubl, C ; pts2: B, beta2, gamma2, delta2 (Jacobian standard form).  Four warps, one pairing each; warp 0
-// then forms the right-hand side with two warp-wide F_q^12 products and compares.
-__global__ void __launch_bounds__(128) k_groth16_verify(const Fq* pts1, const Fq2* pts2, int* ok, int* err) {
-  __shared__ wp::Ws wss[4];
+// Warp w pairs g1 with g2 (Jacobian standard form), in the order A/B, alpha/beta, icPubl/gamma, C/delta.  Four warps, one
+// pairing each; warp 0 then forms the right-hand side with two warp-wide F_q^12 products and compares.
+__device__ __forceinline__ void groth16_verify_block(wp::Ws (&wss)[4], const Fq* g1, const Fq2* g2, int* ok, int* err) {
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
   wp::Ws& ws = wss[warp];
   F2::B px, py;
   F2 qx, qy;
-  if (warp_pairing_inputs(ws, pts1 + 3 * warp, pts2 + 3 * warp, px, py, qx, qy, err)) wp::pairing(ws, px, py, qx, qy);
+  if (warp_pairing_inputs(ws, g1, g2, px, py, qx, qy, err)) wp::pairing(ws, px, py, qx, qy);
   else wp::f12_set_one(ws, wp::RF);
   __syncthreads();
   if (warp == 0) {
@@ -884,6 +884,22 @@ __global__ void __launch_bounds__(128) k_groth16_verify(const Fq* pts1, const Fq
     const unsigned all = __ballot_sync(0xffffffffu, same);
     if (lane == 0) *ok = all == 0xffffffffu ? 1 : 0;
   }
+}
+// pts1: A, alpha1, icPubl, C ; pts2: B, beta2, gamma2, delta2
+__global__ void __launch_bounds__(128) k_groth16_verify(const Fq* pts1, const Fq2* pts2, int* ok, int* err) {
+  __shared__ wp::Ws wss[4];
+  const uint32_t warp = threadIdx.x >> 5;
+  groth16_verify_block(wss, pts1 + 3 * warp, pts2 + 3 * warp, ok, err);
+}
+// The same check for proof idx[b] of a batch in block b: vk2 = beta2, gamma2, delta2; icp = the proofs' icPubl.
+__global__ void __launch_bounds__(128) k_vb_verify_each(const Fq* A, const Fq2* B, const Fq* C, const Fq* icp, const Fq* alpha,
+                                                        const Fq2* vk2, const uint32_t* idx, int* ok, int* err) {
+  __shared__ wp::Ws wss[4];
+  const uint32_t warp = threadIdx.x >> 5;
+  const size_t i = idx[blockIdx.x];
+  const Fq* g1 = warp == 0 ? A + 3 * i : (warp == 1 ? alpha : (warp == 2 ? icp + 3 * i : C + 3 * i));
+  const Fq2* g2 = warp == 0 ? B + 3 * i : vk2 + 3 * (warp - 1);
+  groth16_verify_block(wss, g1, g2, ok + blockIdx.x, err);
 }
 // icPubl = IC[0] + sum publicSignals[i] * IC[i+1] (groth16.go:283-286).  The products are independent: one half-warp each,
 // with the GLV split of prove_host.cuh (128 doublings + ~12 additions deep instead of the 254 + ~127 of MulScalar's
@@ -994,12 +1010,192 @@ int groth16_verify_host(const uint64_t* ic, size_t n_ic, const uint64_t* alpha1,
   return check_err_flag<Fq>("groth16_verify");
 }
 
+// groth16.VerifyProof for nproofs proofs under one key (include/b200snark.h b200_groth16_verify_batch).  The proofs the
+// reference pairs bilinearly enter ONE aggregated check (N + 3 Miller loops, one final exponentiation); the others, and every
+// proof of a batch whose aggregated check fails, run the four-pairing check of b200_groth16_verify one block per proof.
+// A failed check verifies its proofs one by one rather than bisecting: that is the cost of the four-pairing route, paid
+// only when a batch holds a bad proof, and every verdict is then the single verifier's own.
+constexpr size_t kMillerThreads = 16384;   // chunk = ceil(pairs / this): longer chunks share one squaring among more pairs
+int groth16_verify_batch_host(const uint64_t* ic, size_t n_ic, const uint64_t* alpha1, const uint64_t* beta2,
+                              const uint64_t* gamma2, const uint64_t* delta2, size_t n, const uint64_t* pi_a,
+                              const uint64_t* pi_b, const uint64_t* pi_c, const uint64_t* pub, size_t npub,
+                              const uint64_t* rho, int* ok, uint64_t* stats) {
+  if (!ic || !alpha1 || !beta2 || !gamma2 || !delta2 || !pi_a || !pi_b || !pi_c || !rho || !ok || (npub && !pub) || n == 0)
+    return fail(B200_EINVAL, "groth16_verify_batch: null pointer or no proofs");
+  if (n_ic < npub + 1) return fail(B200_EINVAL, "groth16_verify_batch: len(IC) < len(publicSignals) + 1");
+  if (n > (1u << 26)) return fail(B200_EINVAL, "groth16_verify_batch: more than 2^26 proofs");
+  for (size_t i = 0; i < n; i++)
+    if (!rho[2 * i] && !rho[2 * i + 1]) return fail(B200_EINVAL, "groth16_verify_batch: rho[%zu] = 0", i);
+  // the verification key, flagged as b200_groth16_verify flags it
+  auto g1_range = [](const uint64_t* p) {
+    for (int k = 0; k < 3; k++) {
+      Fq v;
+      std::memcpy(&v, p + 4 * k, sizeof v);
+      if (v.geq_modulus()) return true;
+    }
+    return false;
+  };
+  auto g2_range = [&](const uint64_t* p) { return g1_range(p) || g1_range(p + 12); };
+  auto g2_inf = [](const uint64_t* p) { return !(p[16] | p[17] | p[18] | p[19] | p[20] | p[21] | p[22] | p[23]); };
+  int vkf = (g1_range(alpha1) || g2_range(beta2)) ? 1 : (g2_inf(beta2) ? 8 : 0);
+  for (const uint64_t* g : {gamma2, delta2}) vkf |= g2_range(g) ? 1 : (g2_inf(g) ? 8 : 0);
+  for (size_t j = 0; j <= npub; j++) vkf |= g1_range(ic + 12 * j) ? 1 : 0;
+  if (vkf & 8) return fail(B200_EINVAL, "groth16_verify_batch: q1[2] != Fq2.One() (verification key G2 point at infinity)");
+  if (vkf) return fail(B200_ERANGE, "groth16_verify_batch: verification key coordinate >= q");
+  std::vector<int> st(n, 0);   // a public signal >= r: what b200_groth16_verify returns before any pairing
+  for (size_t i = 0; i < n; i++)
+    for (size_t j = 0; j < npub; j++)
+      if (fr_load_std(pub + 4 * (i * npub + j)).geq_modulus()) st[i] = B200_ERANGE;
+  const size_t np = n + 3;
+  DevBuf dic, dalpha, dvk2, dA, dB, dC, dpub, drho, dst, dterms, dicp, dic_aff, dg2_aff, dbad, dpairs, drc, dric, dsum, dT, df,
+      dfe, dres, dalpha_gs, dalpha_term;
+  CU(dic.alloc((npub + 1) * 3 * sizeof(Fq)));
+  CU(dalpha.alloc(2 * 3 * sizeof(Fq)));
+  CU(dvk2.alloc(3 * 3 * sizeof(Fq2)));
+  CU(dA.alloc(n * 3 * sizeof(Fq)));
+  CU(dB.alloc(n * 3 * sizeof(Fq2)));
+  CU(dC.alloc(n * 3 * sizeof(Fq)));
+  CU(dpub.alloc(std::max<size_t>(n * npub, 1) * 4 * sizeof(uint64_t)));
+  CU(drho.alloc(n * 2 * sizeof(uint64_t)));
+  CU(dst.alloc(n * sizeof(int)));
+  CU(dterms.alloc(std::max<size_t>(n * npub, 1) * sizeof(Jacobian<Fq>)));
+  CU(dicp.alloc(n * 3 * sizeof(Fq)));
+  CU(dic_aff.alloc((npub + 1) * sizeof(Affine<Fq>)));
+  CU(dg2_aff.alloc(3 * sizeof(Affine<Fq2>)));
+  CU(dbad.alloc(sizeof(int)));
+  CU(dpairs.alloc(np * sizeof(vb::Pair)));
+  CU(drc.alloc(n * sizeof(XYZZ<Fq>)));
+  CU(dric.alloc(n * sizeof(XYZZ<Fq>)));
+  cudaStream_t s = g_stream;
+  CU(cudaMemcpyAsync(dic.p, ic, (npub + 1) * 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dalpha.p, alpha1, 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));   // [alpha, alpha]: k_ic_terms reads slot 1
+  CU(cudaMemcpyAsync(dalpha.as<Fq>() + 3, alpha1, 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.as<Fq2>(), beta2, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.as<Fq2>() + 3, gamma2, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.as<Fq2>() + 6, delta2, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dA.p, pi_a, n * 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dB.p, pi_b, n * 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dC.p, pi_c, n * 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  if (npub) CU(cudaMemcpyAsync(dpub.p, pub, n * npub * 4 * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(drho.p, rho, n * 2 * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dst.p, st.data(), n * sizeof(int), cudaMemcpyHostToDevice, s));
+  CU(cudaMemsetAsync(dbad.p, 0, sizeof(int), s));
+  // 1. per-proof preparation
+  vb::k_vb_vk<<<1, 32, 0, s>>>(dic.as<Fq>(), (uint32_t)(npub + 1), dalpha.as<Fq>(), dvk2.as<Fq2>(), dic_aff.as<Affine<Fq>>(),
+                               dg2_aff.as<Affine<Fq2>>(), dbad.as<int>());
+  if (npub) vb::k_vb_ic_terms<<<nblk(n * npub, 64), 64, 0, s>>>(dic_aff.as<Affine<Fq>>(), dpub.as<uint64_t>(), n, npub, dterms.as<Jacobian<Fq>>());
+  vb::k_vb_ic_sum<<<nblk(n, 64), 64, 0, s>>>(dic.as<Fq>(), dterms.as<Jacobian<Fq>>(), n, npub, dicp.as<Fq>());
+  vb::k_vb_prepare<<<nblk(n, 64), 64, 0, s>>>(dA.as<Fq>(), dB.as<Fq2>(), dC.as<Fq>(), dicp.as<Fq>(), drho.as<uint64_t>(), n,
+                                              dst.as<int>(), dpairs.as<vb::Pair>(), drc.as<XYZZ<Fq>>(), dric.as<XYZZ<Fq>>());
+  CU(cudaGetLastError());
+  int vk_bad = 0;
+  CU(cudaMemcpyAsync(st.data(), dst.p, n * sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&vk_bad, dbad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (vk_bad) return fail(B200_EINVAL, "groth16_verify_batch: verification key point off the curve, or outside G2");
+  std::vector<uint32_t> each;
+  uint64_t rho_sum[4] = {0, 0, 0, 0};   // sum of < 2^26 128-bit values: < 2^154 < r, no reduction
+  size_t n_agg = 0;
+  for (size_t i = 0; i < n; i++) {
+    if (st[i] == vb::kEach) each.push_back((uint32_t)i);
+    if (st[i] != vb::kAgg) continue;
+    n_agg++;
+    unsigned __int128 c = (unsigned __int128)rho_sum[0] + rho[2 * i];
+    rho_sum[0] = (uint64_t)c;
+    c = (c >> 64) + rho_sum[1] + rho[2 * i + 1];
+    rho_sum[1] = (uint64_t)c;
+    c = (c >> 64) + rho_sum[2];
+    rho_sum[2] = (uint64_t)c;
+  }
+  uint64_t st_stats[4] = {n_agg, 0, 0, 0};
+  bool agg_ok = false;
+  if (n_agg) {
+    // 2. reductions: -(sum rho) alpha by the GLV half-warp of k_ic_terms, sum rho C and sum rho icPubl by tree sums
+    static const uint64_t kR[4] = {0x43e1f593f0000001ULL, 0x2833e84879b97091ULL, 0xb85045b68181585dULL, 0x30644e72e131a029ULL};
+    uint64_t neg[4];
+    unsigned __int128 br = 0;
+    for (int k = 0; k < 4; k++) {
+      unsigned __int128 d = (unsigned __int128)kR[k] - rho_sum[k] - (uint64_t)br;
+      neg[k] = (uint64_t)d;
+      br = (d >> 64) & 1;
+    }
+    GlvScalar gs;
+    if (glv_decompose(fr_load_std(neg), gs.k, gs.neg)) return fail(B200_EINVAL, "groth16_verify_batch: GLV decomposition out of range");
+    CU(dalpha_gs.alloc(sizeof(GlvScalar)));
+    CU(dalpha_term.alloc(sizeof(Jacobian<Fq>)));
+    CU(cudaMemcpyAsync(dalpha_gs.p, &gs, sizeof(GlvScalar), cudaMemcpyHostToDevice, s));
+    k_ic_terms<<<1, 32, 0, s>>>(dalpha.as<Fq>(), dalpha_gs.as<GlvScalar>(), 1, dalpha_term.as<Jacobian<Fq>>(), g_d_err);
+    const uint32_t kSum = 32;
+    size_t levels = 0;   // every level of both sums gets its own slots
+    for (size_t m = n; m > 1; m = nblk(m, kSum)) levels += nblk(m, kSum);
+    CU(dsum.alloc(std::max<size_t>(2 * levels, 1) * sizeof(XYZZ<Fq>)));
+    XYZZ<Fq>* sums[2] = {dric.as<XYZZ<Fq>>(), drc.as<XYZZ<Fq>>()};
+    XYZZ<Fq>* slot = dsum.as<XYZZ<Fq>>();
+    for (int k = 0; k < 2; k++)
+      for (size_t m = n; m > 1; m = nblk(m, kSum)) {
+        vb::k_vb_sum<<<nblk(nblk(m, kSum), 64), 64, 0, s>>>(sums[k], m, kSum, slot);
+        sums[k] = slot;
+        slot += nblk(m, kSum);
+      }
+    CU(dres.alloc(2 * sizeof(int)));
+    vb::k_vb_tail<<<1, 32, 0, s>>>(dalpha_term.as<Jacobian<Fq>>(), sums[0], sums[1], dg2_aff.as<Affine<Fq2>>(),
+                                   dpairs.as<vb::Pair>() + n, dres.as<int>());
+    // 3. multi-Miller loop, 4. product tree and one final exponentiation
+    const uint32_t chunk = (uint32_t)std::max<size_t>(1, nblk(np, kMillerThreads));
+    const size_t nth = nblk(np, chunk);
+    CU(dT.alloc(np * sizeof(Jacobian<Fq2>)));
+    CU(df.alloc(nth * sizeof(F12)));
+    CU(dfe.alloc(nblk(nth, 2) * sizeof(F12)));
+    vb::k_vb_miller<<<nblk(nth, 64), 64, 0, s>>>(dpairs.as<vb::Pair>(), np, chunk, dT.as<Jacobian<Fq2>>(), df.as<F12>());
+    F12 *a = df.as<F12>(), *b = dfe.as<F12>();
+    for (size_t m = nth; m > 1; m = nblk(m, 2)) {
+      vb::k_vb_f12_tree<<<nblk(nblk(m, 2), 64), 64, 0, s>>>(a, m, b);
+      std::swap(a, b);
+    }
+    vb::k_vb_final_exp<<<1, 32, 0, s>>>(a, dres.as<int>() + 1, nullptr);
+    CU(cudaGetLastError());
+    int res[2] = {0, 0};
+    CU(cudaMemcpyAsync(res, dres.p, sizeof res, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    agg_ok = res[1] == 1;
+    st_stats[2] = 1;
+    st_stats[3] = n_agg + (uint64_t)res[0];
+    if (!agg_ok)
+      for (size_t i = 0; i < n; i++)
+        if (st[i] == vb::kAgg) each.push_back((uint32_t)i);
+  }
+  std::vector<int> each_ok(each.size(), 0);
+  if (!each.empty()) {
+    DevBuf didx, dok, derr;
+    CU(didx.alloc(each.size() * sizeof(uint32_t)));
+    CU(dok.alloc(each.size() * sizeof(int)));
+    CU(derr.alloc(sizeof(int)));   // inputs validated above: no flag can be raised
+    CU(cudaMemcpyAsync(didx.p, each.data(), each.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+    k_vb_verify_each<<<(unsigned)each.size(), 128, 0, s>>>(dA.as<Fq>(), dB.as<Fq2>(), dC.as<Fq>(), dicp.as<Fq>(), dalpha.as<Fq>(),
+                                                         dvk2.as<Fq2>(), didx.as<uint32_t>(), dok.as<int>(), derr.as<int>());
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(each_ok.data(), dok.p, each.size() * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    st_stats[1] = each.size();
+    st_stats[3] += 4 * (uint64_t)each.size();
+  }
+  for (size_t i = 0; i < n; i++) ok[i] = st[i] < 0 ? st[i] : (st[i] == vb::kAgg && agg_ok ? 1 : 0);
+  for (size_t k = 0; k < each.size(); k++) ok[each[k]] = each_ok[k];
+  if (stats) std::memcpy(stats, st_stats, sizeof st_stats);
+  return B200_OK;
+}
+
 #else  // experiment builds without the verifier side (ptxas 12.9 crashes on the pairing kernels under -DB200_KARATSUBA)
 int pairing_batch_host(const uint64_t*, const uint64_t*, size_t, uint64_t*) { return fail(B200_EINVAL, "pairing: not in this build variant"); }
 int fq12_mul_batch_host(const uint64_t*, const uint64_t*, size_t, uint64_t*) { return fail(B200_EINVAL, "fq12_mul: not in this build variant"); }
 int groth16_verify_host(const uint64_t*, size_t, const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*,
                         const uint64_t*, const uint64_t*, const uint64_t*, size_t, int*) {
   return fail(B200_EINVAL, "groth16_verify: not in this build variant");
+}
+int groth16_verify_batch_host(const uint64_t*, size_t, const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*, size_t,
+                              const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*, size_t, const uint64_t*, int*,
+                              uint64_t*) {
+  return fail(B200_EINVAL, "groth16_verify_batch: not in this build variant");
 }
 #endif
 
@@ -1261,6 +1457,13 @@ int b200_groth16_verify(const uint64_t* ic, size_t n_ic, const uint64_t alpha1[1
                         const uint64_t pi_b[24], const uint64_t pi_c[12], const uint64_t* public_signals, size_t n_public,
                         int* ok) {
   B200_API_BODY(groth16_verify_host(ic, n_ic, alpha1, beta2, gamma2, delta2, pi_a, pi_b, pi_c, public_signals, n_public, ok))
+}
+int b200_groth16_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t alpha1[12], const uint64_t beta2[24],
+                              const uint64_t gamma2[24], const uint64_t delta2[24], size_t nproofs, const uint64_t* pi_a,
+                              const uint64_t* pi_b, const uint64_t* pi_c, const uint64_t* public_signals, size_t n_public,
+                              const uint64_t* rho, int* ok, uint64_t stats[4]) {
+  B200_API_BODY(groth16_verify_batch_host(ic, n_ic, alpha1, beta2, gamma2, delta2, nproofs, pi_a, pi_b, pi_c, public_signals,
+                                          n_public, rho, ok, stats))
 }
 int b200_g1_add_batch(const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out) { B200_API_BODY(group_op_host<Fq>(0, p, q, n, out)) }
 int b200_g1_double_batch(const uint64_t* p, size_t n, uint64_t* out) { B200_API_BODY(group_op_host<Fq>(1, p, nullptr, n, out)) }

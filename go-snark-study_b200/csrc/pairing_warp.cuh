@@ -246,46 +246,11 @@ DEV void pairing_constants(Ws& ws) {
   wsync();
 }
 
-// Pairing of affine Montgomery-form inputs: the value of pairing_affine_t<true> in r[0] (all lanes call; px, py, qx, qy
-// need only be valid on lane 0).
 constexpr int RF = 0, RS = 1;   // accumulator, line value
-DEV void pairing(Ws& ws, const F2::B& px, const F2::B& py, const F2& qx, const F2& qy) {
-  const uint32_t lane = lane_id();
-  if (lane == 0) {
-    ws.px = px;
-    ws.py = py;
-    ws.Q[0] = qx;
-    ws.Q[1] = qy;
-    ws.P[0] = qx;
-    ws.P[1] = qy;
-    ws.P[2] = F2::one();
-    // q1 = pi(Q), q2 = -pi^2(Q)  (bn128.go:238-253, 331-346)
-    const F2 tqx = B200_F2_CONST(TWIST_MUL_BY_Q_X), tqy = B200_F2_CONST(TWIST_MUL_BY_Q_Y);
-    const F2 q1x = tqx * F2{qx.c0, qx.c1.neg()}, q1y = tqy * F2{qy.c0, qy.c1.neg()};
-    ws.Q[2] = q1x;
-    ws.Q[3] = q1y;
-    ws.Q[4] = tqx * F2{q1x.c0, q1x.c1.neg()};
-    ws.Q[5] = (tqy * F2{q1y.c0, q1y.c1.neg()}).neg();
-  }
-  wsync();
-  pairing_constants(ws);
-  f12_set_one(ws, RF);
-  // Miller loop (bn128.go:354-372), the G2 precomputation fused with it
-#pragma unroll 1
-  for (int i = 63; i >= 0; i--) {
-    doubling_step(ws, RS);
-    f12_sqr(ws, RF, RF);
-    f12_mul(ws, RF, RF, RS);
-    if ((pc::LOOP_COUNT_LOW64 >> i) & 1) {
-      addition_step(ws, RS, 0);
-      f12_mul(ws, RF, RF, RS);
-    }
-  }
-  addition_step(ws, RS, 1);
-  f12_mul(ws, RF, RF, RS);
-  addition_step(ws, RS, 2);
-  f12_mul(ws, RF, RF, RS);
-  // final exponentiation, Devegili-Scott-Dahab (pairing.cuh final_exp_fast, same operations)
+
+// r[RF] <- r[RF]^((q^12 - 1) / r): Devegili-Scott-Dahab, the operations of pairing.cuh final_exp_fast.  Needs the Frobenius
+// constants in ws.fc (pairing_constants) and uses registers 1..11 as scratch.
+DEV void final_exp(Ws& ws) {
   enum { M = 2, MU = 3, MU2 = 4, MU3 = 5, Y0 = 6, Y2 = 7, Y3 = 8, Y4 = 9, Y6 = 10, T0 = 11, T1 = 1 };
   f12_inverse(ws, T0, RF);
   f12_conj(ws, M, RF);
@@ -325,6 +290,47 @@ DEV void pairing(Ws& ws, const F2::B& px, const F2::B& py, const F2& qx, const F
   f12_mul(ws, T1, T1, Y0);               // t1 = t1 y0
   f12_sqr(ws, T0, T0);
   f12_mul(ws, RF, T0, T1);
+}
+
+// Pairing of affine Montgomery-form inputs: the value of pairing_affine_t<true> in r[0] (all lanes call; px, py, qx, qy
+// need only be valid on lane 0).
+DEV void pairing(Ws& ws, const F2::B& px, const F2::B& py, const F2& qx, const F2& qy) {
+  const uint32_t lane = lane_id();
+  if (lane == 0) {
+    ws.px = px;
+    ws.py = py;
+    ws.Q[0] = qx;
+    ws.Q[1] = qy;
+    ws.P[0] = qx;
+    ws.P[1] = qy;
+    ws.P[2] = F2::one();
+    // q1 = pi(Q), q2 = -pi^2(Q)  (bn128.go:238-253, 331-346)
+    const F2 tqx = B200_F2_CONST(TWIST_MUL_BY_Q_X), tqy = B200_F2_CONST(TWIST_MUL_BY_Q_Y);
+    const F2 q1x = tqx * F2{qx.c0, qx.c1.neg()}, q1y = tqy * F2{qy.c0, qy.c1.neg()};
+    ws.Q[2] = q1x;
+    ws.Q[3] = q1y;
+    ws.Q[4] = tqx * F2{q1x.c0, q1x.c1.neg()};
+    ws.Q[5] = (tqy * F2{q1y.c0, q1y.c1.neg()}).neg();
+  }
+  wsync();
+  pairing_constants(ws);
+  f12_set_one(ws, RF);
+  // Miller loop (bn128.go:354-372), the G2 precomputation fused with it
+#pragma unroll 1
+  for (int i = 63; i >= 0; i--) {
+    doubling_step(ws, RS);
+    f12_sqr(ws, RF, RF);
+    f12_mul(ws, RF, RF, RS);
+    if ((pc::LOOP_COUNT_LOW64 >> i) & 1) {
+      addition_step(ws, RS, 0);
+      f12_mul(ws, RF, RF, RS);
+    }
+  }
+  addition_step(ws, RS, 1);
+  f12_mul(ws, RF, RF, RS);
+  addition_step(ws, RS, 2);
+  f12_mul(ws, RF, RF, RS);
+  final_exp(ws);
 }
 
 }  // namespace wp

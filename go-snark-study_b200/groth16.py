@@ -205,3 +205,43 @@ def VerifyProof(vk, proof, publicSignals, debug=False):
     if debug:
         print("✓ groth16 verification passed" if ok.value else "❌ groth16 verification not passed")
     return bool(ok.value)
+
+
+def _rand_rho():
+    """A uniformly random non-zero 128-bit batching scalar (16 bytes from the OS CSPRNG, 0 rejected)."""
+    while True:
+        v = int.from_bytes(secrets.token_bytes(16), "little")
+        if v:
+            return v
+
+
+def VerifyProofBatch(vk, proofs, publicSignals, rho=None, stats=None):
+    """VerifyProof for every proofs[i] with publicSignals[i] under one vk, as one random linear combination on the GPU
+    (b200_groth16_verify_batch): one Miller loop per proof, three for the key, one final exponentiation.  rho: one non-zero
+    128-bit scalar per proof, secret from whoever made the proofs; drawn here with ``secrets`` when None.  Returns a
+    list of bools, False wherever VerifyProof would return False or raise.  ``stats`` (a list) receives the library's
+    counters: proofs in the aggregated check, proofs verified one by one, aggregated checks run, Miller loops run."""
+    n = len(proofs)
+    if len(publicSignals) != n:
+        raise ValueError("VerifyProofBatch: one publicSignals list per proof")
+    if n == 0:
+        return []
+    npub = len(publicSignals[0])
+    if any(len(p) != npub for p in publicSignals):
+        raise ValueError("VerifyProofBatch: every proof needs the same number of public signals")
+    if rho is None:
+        rho = [_rand_rho() for _ in range(n)]
+    if len(rho) != n or any(not 0 < int(r) < (1 << 128) for r in rho):
+        raise ValueError("VerifyProofBatch: rho must be n non-zero 128-bit integers")
+    pub = ints_to_limbs([reduce_scalar(x) for sig in publicSignals for x in sig]) if npub else np.zeros((1, 4), dtype=np.uint64)
+    rl = ints_to_limbs(rho, 2)
+    ok = np.zeros(n, dtype=np.int32)
+    st = np.zeros(4, dtype=np.uint64)
+    check(lib().b200_groth16_verify_batch(ptr(_flatten_g1(vk["IC"])), len(vk["IC"]), ptr(_flatten_g1([vk["G1"]["Alpha"]])),
+                                          ptr(_flatten_g2([vk["G2"]["Beta"]])), ptr(_flatten_g2([vk["G2"]["Gamma"]])),
+                                          ptr(_flatten_g2([vk["G2"]["Delta"]])), n,
+                                          ptr(_flatten_g1([p["PiA"] for p in proofs])), ptr(_flatten_g2([p["PiB"] for p in proofs])),
+                                          ptr(_flatten_g1([p["PiC"] for p in proofs])), ptr(pub), npub, ptr(rl), ptr(ok), ptr(st)))
+    if stats is not None:
+        stats[:] = [int(x) for x in st]
+    return [bool(v == 1) for v in ok]

@@ -260,6 +260,23 @@ int b200_groth16_verify(const uint64_t* ic, size_t n_ic, const uint64_t alpha1[1
                         const uint64_t gamma2[24], const uint64_t delta2[24], const uint64_t pi_a[12],
                         const uint64_t pi_b[24], const uint64_t pi_c[12], const uint64_t* public_signals, size_t n_public,
                         int* ok);
+/* Verify nproofs Groth16 proofs under ONE verification key (groth16.VerifyProof, groth16/groth16.go:281-305, per proof).
+ * pi_a: nproofs x 12 u64, pi_b: nproofs x 24, pi_c: nproofs x 12, public_signals: nproofs x n_public x 4 (row-major),
+ * rho: nproofs x 2 u64 — the caller's secret, uniformly random, non-zero 128-bit batching scalars (like r, s of the prove
+ * calls, drawn by the caller; a prover who knows them can make invalid proofs cancel).  ok[i] = 1 / 0, or the negative
+ * code b200_groth16_verify would return for proof i alone.  stats (may be NULL) = { proofs in the aggregated check,
+ * proofs verified one by one, aggregated checks run, Miller loops run }.
+ * The proofs that pair bilinearly are checked together: prod e(rho_i A_i, B_i) * e(-(sum rho_i) alpha, beta) *
+ * e(-sum rho_i icPubl_i, gamma) * e(-sum rho_i C_i, delta) == 1, N + 3 Miller loops and one final exponentiation (a false
+ * accept has probability <= 2^-128 over rho).  A, C or icPubl at infinity, A or C off the curve, B off the twist or outside
+ * G2 are verified one by one, as is every proof of a batch whose aggregated check fails.  Call-level errors, ok[] untouched:
+ * null pointers, nproofs == 0, n_ic < n_public + 1, a rho_i == 0 (B200_EINVAL); a verification-key coordinate >= q
+ * (B200_ERANGE) or G2 point at infinity (B200_EINVAL); alpha at infinity, a vk point off the curve or outside G2 (EINVAL). */
+int b200_groth16_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t alpha1[12], const uint64_t beta2[24],
+                              const uint64_t gamma2[24], const uint64_t delta2[24], size_t nproofs,
+                              const uint64_t* pi_a, const uint64_t* pi_b, const uint64_t* pi_c,
+                              const uint64_t* public_signals, size_t n_public, const uint64_t* rho,
+                              int* ok, uint64_t stats[4]);
 
 /* ---- dense QAP API upstream of GenerateProofs (small n; the prove path consumes px) ---- */
 /* PolynomialField.R1CSToQAP (r1csqap/r1csqap.go:161-188).  a, b, c: n x m row-major R1CS matrices (coefficients
