@@ -101,6 +101,19 @@ def build_host_verify_batch(force=False):
     return target
 
 
+def build_host_pinocchio_verify_batch(force=False):
+    """g++ build of the Pinocchio verification kernels of csrc/verify_batch_pinocchio.cuh over tests/host/host_stub (CPU
+    test vehicle, tests/test_host_pinocchio_verify_batch.py)."""
+    os.makedirs(LIBDIR, exist_ok=True)
+    target = os.path.join(LIBDIR, "libb200_host_pinocchio_verify_batch.so")
+    if not force and not _newer(target, _all_sources() + [os.path.join(HOSTTEST, "host_stub", "cuda_runtime.h")]):
+        return target
+    cmd = ["g++", "-O2", "-std=c++17", "-pthread", "-x", "c++", "-shared", "-fPIC", "-Wno-psabi", "-I", os.path.join(HOSTTEST, "host_stub"),
+           "-I", HOSTTEST, "-I", CSRC, "-o", target, os.path.join(HOSTTEST, "host_pinocchio_verify_batch_test.cpp")]
+    _run(cmd)
+    return target
+
+
 def build_shard_partition(force=False):
     """g++ build of csrc/shard_partition.h behind a C entry point (CPU test vehicle, tests/test_shard_partition.py)."""
     os.makedirs(LIBDIR, exist_ok=True)

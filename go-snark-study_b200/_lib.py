@@ -79,6 +79,8 @@ _SIGNATURES = {
     "b200_fq12_mul_batch": [_vp, _vp, _sz, _vp],
     "b200_groth16_verify": [_vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.POINTER(_int)],
     "b200_groth16_verify_batch": [_vp, _sz, _vp, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _sz, _vp, _vp, _vp],
+    "b200_pinocchio_verify": [_vp, _sz, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp],
+    "b200_pinocchio_verify_batch": [_vp, _sz, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp],
     "b200_r1cs_to_qap": [_vp, _vp, _vp, _sz, _sz, _vp, _vp, _vp, _vp],
     "b200_combine_polynomials": [_vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp],
     "b200_g1_add_batch": [_vp, _vp, _sz, _vp], "b200_g2_add_batch": [_vp, _vp, _sz, _vp],

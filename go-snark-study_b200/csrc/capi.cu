@@ -27,6 +27,7 @@
 #include "pairing.cuh"
 #include "pairing_warp.cuh"
 #include "verify_batch.cuh"
+#include "verify_batch_pinocchio.cuh"
 #endif
 
 using namespace b200;
@@ -935,6 +936,14 @@ __global__ void k_ic_sum(const Fq* ic, const Jacobian<Fq>* terms, size_t npub, F
 // GPU against the snarkjs golden vk_alfabeta_12 (K8), the bn128_test.go literal and the oracle (tests/test_gpu_verify.py,
 // profiles/r2_notes.md).  The plain routine stays in pairing.cuh as the step-by-step restatement used by the host tests.
 constexpr bool kFastFinalExp = true;
+// n pairings of device inputs (Jacobian standard form) into out (standard form).  auto: a warp per pairing has the 5x shorter
+// latency (3.4 vs 17 ms) and wins up to ~3 500 pairings per call; above that the thread-per-pairing kernel keeps more
+// pairings resident and has twice the throughput (462 k vs 204 k pairings/s at 2^16)
+void pairing_enqueue(const Fq* g1, const Fq2* g2, size_t n, Fq2* out, cudaStream_t st) {
+  const bool thread_kernel = g_pairing_kernel == 1 || (g_pairing_kernel == 0 && n > 2048);
+  if (thread_kernel) k_pairing_batch<kFastFinalExp><<<nblk(n, 32), 32, 0, st>>>(g1, g2, n, out, g_d_err);
+  else k_pairing_batch_warp<<<nblk(n, kPairWarps), 32 * kPairWarps, 0, st>>>(g1, g2, n, out, g_d_err);
+}
 int pairing_batch_host(const uint64_t* g1, const uint64_t* g2, size_t n, uint64_t* out) {
   if (!g1 || !g2 || !out) return fail(B200_EINVAL, "pairing_batch: null pointer");
   if (n == 0) return B200_OK;
@@ -944,11 +953,7 @@ int pairing_batch_host(const uint64_t* g1, const uint64_t* g2, size_t n, uint64_
   CU(dout.alloc(n * 6 * sizeof(Fq2)));
   CU(cudaMemcpyAsync(d1.p, g1, n * 3 * sizeof(Fq), cudaMemcpyHostToDevice, g_stream));
   CU(cudaMemcpyAsync(d2.p, g2, n * 3 * sizeof(Fq2), cudaMemcpyHostToDevice, g_stream));
-  // auto: a warp per pairing has the 5x shorter latency (3.4 vs 17 ms) and wins up to ~3 500 pairings per call; above that the
-  // thread-per-pairing kernel keeps more pairings resident and has twice the throughput (462 k vs 204 k pairings/s at 2^16)
-  const bool thread_kernel = g_pairing_kernel == 1 || (g_pairing_kernel == 0 && n > 2048);
-  if (thread_kernel) k_pairing_batch<kFastFinalExp><<<nblk(n, 32), 32, 0, g_stream>>>(d1.as<Fq>(), d2.as<Fq2>(), n, dout.as<Fq2>(), g_d_err);
-  else k_pairing_batch_warp<<<nblk(n, kPairWarps), 32 * kPairWarps, 0, g_stream>>>(d1.as<Fq>(), d2.as<Fq2>(), n, dout.as<Fq2>(), g_d_err);
+  pairing_enqueue(d1.as<Fq>(), d2.as<Fq2>(), n, dout.as<Fq2>(), g_stream);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(out, dout.p, n * 6 * sizeof(Fq2), cudaMemcpyDeviceToHost, g_stream));
   return check_err_flag<Fq>("pairing_batch");
@@ -1185,6 +1190,228 @@ int groth16_verify_batch_host(const uint64_t* ic, size_t n_ic, const uint64_t* a
   return B200_OK;
 }
 
+// ---- Pinocchio verification (snark.VerifyProof, snark.go:292-372): one proof, and N proofs under one key ----
+// the generator of G2 (bn128.go:57-83), Jacobian standard form
+constexpr uint64_t kG2Gen[24] = {
+    0x46debd5cd992f6edULL, 0x674322d4f75edaddULL, 0x426a00665e5c4479ULL, 0x1800deef121f1e76ULL,
+    0x97e485b7aef312c2ULL, 0xf1aa493335a9e712ULL, 0x7260bfb731fb5d25ULL, 0x198e9393920d483aULL,
+    0x4ce6cc0166fa7daaULL, 0xe3d1e7690c43d37bULL, 0x4aab71808dcb408fULL, 0x12c85ea5db8c6debULL,
+    0x55acdadcd122975bULL, 0xbc4b313370b38ef3ULL, 0xec9e99ad690c3395ULL, 0x090689d0585ff075ULL,
+    1, 0, 0, 0, 0, 0, 0, 0};
+bool fq_any_geq_q(const uint64_t* p, size_t nfe) {
+  for (size_t k = 0; k < nfe; k++) {
+    Fq v;
+    std::memcpy(&v, p + 4 * k, sizeof v);
+    if (v.geq_modulus()) return true;
+  }
+  return false;
+}
+bool g2_at_infinity(const uint64_t* p) { return !(p[16] | p[17] | p[18] | p[19] | p[20] | p[21] | p[22] | p[23]); }
+// The verification key's code: a G2 point at infinity (B200_EINVAL, before anything else) or a coordinate >= q (B200_ERANGE)
+// among IC[0..npub], vk_g1 and vk_g2.
+int pv_vk_code(const uint64_t* ic, size_t npub, const uint64_t* vk_g1, const uint64_t* vk_g2) {
+  for (int k = 0; k < 5; k++)
+    if (g2_at_infinity(vk_g2 + 24 * k)) return B200_EINVAL;
+  if (fq_any_geq_q(ic, 3 * (npub + 1)) || fq_any_geq_q(vk_g1, 6) || fq_any_geq_q(vk_g2, 30)) return B200_ERANGE;
+  return B200_OK;
+}
+// The twelve pairings and five checks of snark.VerifyProof for m proofs on the device: proof idx[b] (b when idx is null).
+// P, B: the proofs' G1 points and PiB; vkx: their IC sums; vk1, vk2 as k_pv_pairs reads them.  failed (host, m ints): 0 or
+// the first failing check.  Inputs are validated by the caller.
+int pv_check(const Fq* P, const Fq2* B, const Fq* vkx, const Fq* vk1, const Fq2* vk2, const uint32_t* idx, size_t m,
+             int* failed) {
+  DevBuf d1, d2, de, df;
+  CU(d1.alloc(12 * m * 3 * sizeof(Fq)));
+  CU(d2.alloc(12 * m * 3 * sizeof(Fq2)));
+  CU(de.alloc(12 * m * 6 * sizeof(Fq2)));
+  CU(df.alloc(m * sizeof(int)));
+  cudaStream_t s = g_stream;
+  pv::k_pv_pairs<<<nblk(m, 64), 64, 0, s>>>(P, B, vkx, vk1, vk2, idx, m, d1.as<Fq>(), d2.as<Fq2>());
+  pairing_enqueue(d1.as<Fq>(), d2.as<Fq2>(), 12 * m, de.as<Fq2>(), s);
+  pv::k_pv_compare<<<nblk(m, 64), 64, 0, s>>>(de.as<Fq2>(), m, df.as<int>());
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(failed, df.p, m * sizeof(int), cudaMemcpyDeviceToHost, s));
+  return check_err_flag<Fq>("pinocchio_verify");
+}
+
+int pinocchio_verify_host(const uint64_t* ic, size_t n_ic, const uint64_t* vk_g1, const uint64_t* vk_g2,
+                          const uint64_t* proof_g1, const uint64_t* pi_b, const uint64_t* pub, size_t npub, int* ok,
+                          int* failed_check) {
+  if (!ic || !vk_g1 || !vk_g2 || !proof_g1 || !pi_b || !ok || (npub && !pub)) return fail(B200_EINVAL, "pinocchio_verify: null pointer");
+  if (n_ic < npub + 1) return fail(B200_EINVAL, "pinocchio_verify: len(IC) < len(publicSignals) + 1");
+  const int vkc = pv_vk_code(ic, npub, vk_g1, vk_g2);
+  if (vkc == B200_EINVAL || g2_at_infinity(pi_b))
+    return fail(B200_EINVAL, "pinocchio_verify: q1[2] != Fq2.One() (G2 point at infinity; the reference panics, bn128.go:238-241)");
+  if (vkc || fq_any_geq_q(proof_g1, 21) || fq_any_geq_q(pi_b, 6)) return fail(B200_ERANGE, "pinocchio_verify: point coordinate >= q");
+  std::vector<GlvScalar> gs(npub ? npub : 1);
+  for (size_t i = 0; i < npub; i++) {
+    Fr v = fr_load_std(pub + 4 * i);
+    if (v.geq_modulus()) return fail(B200_ERANGE, "pinocchio_verify: scalar / coefficient >= r");
+    if (glv_decompose(v, gs[i].k, gs[i].neg)) return fail(B200_EINVAL, "pinocchio_verify: GLV decomposition out of range");
+  }
+  DevBuf dic, dsig, dterms, dvkx, dP, dB, dvk1, dvk2;
+  CU(dic.alloc((npub + 1) * 3 * sizeof(Fq)));
+  CU(dsig.alloc(gs.size() * sizeof(GlvScalar)));
+  CU(dterms.alloc(gs.size() * sizeof(Jacobian<Fq>)));
+  CU(dvkx.alloc(3 * sizeof(Fq)));
+  CU(dP.alloc(21 * sizeof(Fq)));
+  CU(dB.alloc(3 * sizeof(Fq2)));
+  CU(dvk1.alloc(6 * sizeof(Fq)));
+  CU(dvk2.alloc(18 * sizeof(Fq2)));
+  cudaStream_t s = g_stream;
+  CU(cudaMemcpyAsync(dic.p, ic, (npub + 1) * 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  if (npub) CU(cudaMemcpyAsync(dsig.p, gs.data(), npub * sizeof(GlvScalar), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dP.p, proof_g1, 21 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dB.p, pi_b, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk1.p, vk_g1, 6 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.p, kG2Gen, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.as<Fq2>() + 3, vk_g2, 15 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  if (npub) k_ic_terms<<<(unsigned)((npub + 1) / 2), 32, 0, s>>>(dic.as<Fq>(), dsig.as<GlvScalar>(), npub, dterms.as<Jacobian<Fq>>(), g_d_err);
+  k_ic_sum<<<1, 32, 0, s>>>(dic.as<Fq>(), dterms.as<Jacobian<Fq>>(), npub, dvkx.as<Fq>(), g_d_err);
+  int failed = -1;
+  if (int rc = pv_check(dP.as<Fq>(), dB.as<Fq2>(), dvkx.as<Fq>(), dvk1.as<Fq>(), dvk2.as<Fq2>(), nullptr, 1, &failed)) return rc;
+  *ok = failed == 0 ? 1 : 0;
+  if (failed_check) *failed_check = failed;
+  return B200_OK;
+}
+
+// snark.VerifyProof for nproofs proofs under one key (include/b200snark.h b200_pinocchio_verify_batch).  The proofs the
+// reference pairs bilinearly enter ONE aggregated check (N + 6 Miller loops, one final exponentiation, verify_batch_pinocchio.cuh);
+// the others, and every proof of a batch whose aggregated check fails, run the twelve pairings of b200_pinocchio_verify.
+// As for Groth16, a failed check verifies its proofs one by one rather than bisecting.
+int pinocchio_verify_batch_host(const uint64_t* ic, size_t n_ic, const uint64_t* vk_g1, const uint64_t* vk_g2, size_t n,
+                                const uint64_t* proofs_g1, const uint64_t* pi_b, const uint64_t* pub, size_t npub,
+                                const uint64_t* rho, int* ok, uint64_t* stats) {
+  if (!ic || !vk_g1 || !vk_g2 || !proofs_g1 || !pi_b || !rho || !ok || (npub && !pub) || n == 0)
+    return fail(B200_EINVAL, "pinocchio_verify_batch: null pointer or no proofs");
+  if (n_ic < npub + 1) return fail(B200_EINVAL, "pinocchio_verify_batch: len(IC) < len(publicSignals) + 1");
+  if (n > (1u << 26)) return fail(B200_EINVAL, "pinocchio_verify_batch: more than 2^26 proofs");
+  for (size_t k = 0; k < 5 * n; k++)
+    if (!rho[2 * k] && !rho[2 * k + 1]) return fail(B200_EINVAL, "pinocchio_verify_batch: rho[%zu][%zu] = 0", k / 5, k % 5);
+  const int vkc = pv_vk_code(ic, npub, vk_g1, vk_g2);
+  if (vkc == B200_EINVAL) return fail(B200_EINVAL, "pinocchio_verify_batch: q1[2] != Fq2.One() (verification key G2 point at infinity)");
+  if (vkc) return fail(B200_ERANGE, "pinocchio_verify_batch: verification key coordinate >= q");
+  std::vector<int> st(n, 0);   // a public signal >= r: B200_ERANGE unless k_pv_prepare finds PiB at infinity
+  for (size_t i = 0; i < n; i++)
+    for (size_t j = 0; j < npub; j++)
+      if (fr_load_std(pub + 4 * (i * npub + j)).geq_modulus()) st[i] = B200_ERANGE;
+  const size_t np = n + 6;
+  DevBuf dic, dvk1, dvk2, dP, dB, dpub, drho, dst, dterms, dvkx, dic_aff, dg1_aff, dg2_aff, dbad, dpts, dqb, dpairs, dsums, dsum,
+      dT, df, dfe, dres;
+  CU(dic.alloc((npub + 1) * 3 * sizeof(Fq)));
+  CU(dvk1.alloc(6 * sizeof(Fq)));
+  CU(dvk2.alloc(18 * sizeof(Fq2)));
+  CU(dP.alloc(n * 21 * sizeof(Fq)));
+  CU(dB.alloc(n * 3 * sizeof(Fq2)));
+  CU(dpub.alloc(std::max<size_t>(n * npub, 1) * 4 * sizeof(uint64_t)));
+  CU(drho.alloc(n * 10 * sizeof(uint64_t)));
+  CU(dst.alloc(n * sizeof(int)));
+  CU(dterms.alloc(std::max<size_t>(n * npub, 1) * sizeof(Jacobian<Fq>)));
+  CU(dvkx.alloc(n * 3 * sizeof(Fq)));
+  CU(dic_aff.alloc((npub + 1) * sizeof(Affine<Fq>)));
+  CU(dg1_aff.alloc(pv::kVkG1 * sizeof(Affine<Fq>)));
+  CU(dg2_aff.alloc(pv::kVkG2 * sizeof(Affine<Fq2>)));
+  CU(dbad.alloc(sizeof(int)));
+  CU(dpts.alloc(n * pv::kPts * sizeof(Affine<Fq>)));
+  CU(dqb.alloc(n * sizeof(Affine<Fq2>)));
+  cudaStream_t s = g_stream;
+  CU(cudaMemcpyAsync(dic.p, ic, (npub + 1) * 3 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk1.p, vk_g1, 6 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.p, kG2Gen, 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dvk2.as<Fq2>() + 3, vk_g2, 15 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dP.p, proofs_g1, n * 21 * sizeof(Fq), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dB.p, pi_b, n * 3 * sizeof(Fq2), cudaMemcpyHostToDevice, s));
+  if (npub) CU(cudaMemcpyAsync(dpub.p, pub, n * npub * 4 * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(drho.p, rho, n * 10 * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dst.p, st.data(), n * sizeof(int), cudaMemcpyHostToDevice, s));
+  CU(cudaMemsetAsync(dbad.p, 0, sizeof(int), s));
+  // 1. the key, vkx_i, per-proof preparation
+  pv::k_pv_vk<<<1, 32, 0, s>>>(dic.as<Fq>(), (uint32_t)(npub + 1), dvk1.as<Fq>(), dvk2.as<Fq2>(), dic_aff.as<Affine<Fq>>(),
+                               dg1_aff.as<Affine<Fq>>(), dg2_aff.as<Affine<Fq2>>(), dbad.as<int>());
+  if (npub) vb::k_vb_ic_terms<<<nblk(n * npub, 64), 64, 0, s>>>(dic_aff.as<Affine<Fq>>(), dpub.as<uint64_t>(), n, npub, dterms.as<Jacobian<Fq>>());
+  vb::k_vb_ic_sum<<<nblk(n, 64), 64, 0, s>>>(dic.as<Fq>(), dterms.as<Jacobian<Fq>>(), n, npub, dvkx.as<Fq>());
+  pv::k_pv_prepare<<<nblk(n, 64), 64, 0, s>>>(dP.as<Fq>(), dB.as<Fq2>(), dvkx.as<Fq>(), n, dst.as<int>(), dpts.as<Affine<Fq>>(),
+                                              dqb.as<Affine<Fq2>>());
+  CU(cudaGetLastError());
+  int vk_bad = 0;
+  CU(cudaMemcpyAsync(st.data(), dst.p, n * sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&vk_bad, dbad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (vk_bad) return fail(B200_EINVAL, "pinocchio_verify_batch: verification key point at infinity, off the curve, or outside G2");
+  std::vector<uint32_t> each;
+  size_t n_agg = 0;
+  for (size_t i = 0; i < n; i++) {
+    if (st[i] == vb::kEach) each.push_back((uint32_t)i);
+    if (st[i] == vb::kAgg) n_agg++;
+  }
+  uint64_t st_stats[4] = {n_agg, 0, 0, 0};
+  bool agg_ok = false;
+  if (n_agg) {
+    // 2. the seven products per proof, tree sums of the six arrays, the six fixed-G2 pairs
+    CU(dpairs.alloc(np * sizeof(vb::Pair)));
+    CU(dsums.alloc(6 * n * sizeof(XYZZ<Fq>)));
+    CU(dres.alloc(2 * sizeof(int)));
+    CU(cudaMemsetAsync(dres.p, 0, 2 * sizeof(int), s));
+    pv::k_pv_products<<<nblk(pv::kProducts * n, 64), 64, 0, s>>>(dpts.as<Affine<Fq>>(), dqb.as<Affine<Fq2>>(), dg1_aff.as<Affine<Fq>>(),
+                                                                 drho.as<uint64_t>(), dst.as<int>(), n, dsums.as<XYZZ<Fq>>(),
+                                                                 dpairs.as<vb::Pair>(), dres.as<int>());
+    const uint32_t kSum = 32;
+    size_t levels = 0;   // every level of every sum gets its own slots
+    for (size_t m = n; m > 1; m = nblk(m, kSum)) levels += nblk(m, kSum);
+    CU(dsum.alloc(std::max<size_t>(6 * levels, 1) * sizeof(XYZZ<Fq>)));
+    pv::Sums6 sums;
+    XYZZ<Fq>* slot = dsum.as<XYZZ<Fq>>();
+    for (int k = 0; k < 6; k++) {
+      const XYZZ<Fq>* cur = dsums.as<XYZZ<Fq>>() + k * n;
+      for (size_t m = n; m > 1; m = nblk(m, kSum)) {
+        vb::k_vb_sum<<<nblk(nblk(m, kSum), 64), 64, 0, s>>>(cur, m, kSum, slot);
+        cur = slot;
+        slot += nblk(m, kSum);
+      }
+      sums.s[k] = cur;
+    }
+    pv::k_pv_tail<<<1, 32, 0, s>>>(sums, dg2_aff.as<Affine<Fq2>>(), dpairs.as<vb::Pair>() + n, dres.as<int>());
+    // 3. multi-Miller loop, 4. product tree and one final exponentiation
+    const uint32_t chunk = (uint32_t)std::max<size_t>(1, nblk(np, kMillerThreads));
+    const size_t nth = nblk(np, chunk);
+    CU(dT.alloc(np * sizeof(Jacobian<Fq2>)));
+    CU(df.alloc(nth * sizeof(F12)));
+    CU(dfe.alloc(nblk(nth, 2) * sizeof(F12)));
+    vb::k_vb_miller<<<nblk(nth, 64), 64, 0, s>>>(dpairs.as<vb::Pair>(), np, chunk, dT.as<Jacobian<Fq2>>(), df.as<F12>());
+    F12 *a = df.as<F12>(), *b = dfe.as<F12>();
+    for (size_t m = nth; m > 1; m = nblk(m, 2)) {
+      vb::k_vb_f12_tree<<<nblk(nblk(m, 2), 64), 64, 0, s>>>(a, m, b);
+      std::swap(a, b);
+    }
+    vb::k_vb_final_exp<<<1, 32, 0, s>>>(a, dres.as<int>() + 1, nullptr);
+    CU(cudaGetLastError());
+    int res[2] = {0, 0};
+    CU(cudaMemcpyAsync(res, dres.p, sizeof res, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    agg_ok = res[1] == 1;
+    st_stats[2] = 1;
+    st_stats[3] = (uint64_t)res[0];
+    if (!agg_ok)
+      for (size_t i = 0; i < n; i++)
+        if (st[i] == vb::kAgg) each.push_back((uint32_t)i);
+  }
+  std::vector<int> failed(each.size(), 0);
+  if (!each.empty()) {
+    DevBuf didx;
+    CU(didx.alloc(each.size() * sizeof(uint32_t)));
+    CU(cudaMemcpyAsync(didx.p, each.data(), each.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+    if (int rc = pv_check(dP.as<Fq>(), dB.as<Fq2>(), dvkx.as<Fq>(), dvk1.as<Fq>(), dvk2.as<Fq2>(), didx.as<uint32_t>(), each.size(),
+                          failed.data()))
+      return rc;
+    st_stats[1] = each.size();
+    st_stats[3] += 12 * (uint64_t)each.size();
+  }
+  for (size_t i = 0; i < n; i++) ok[i] = st[i] < 0 ? st[i] : (st[i] == vb::kAgg && agg_ok ? 1 : 0);
+  for (size_t k = 0; k < each.size(); k++) ok[each[k]] = failed[k] == 0 ? 1 : 0;
+  if (stats) std::memcpy(stats, st_stats, sizeof st_stats);
+  return B200_OK;
+}
+
 #else  // experiment builds without the verifier side (ptxas 12.9 crashes on the pairing kernels under -DB200_KARATSUBA)
 int pairing_batch_host(const uint64_t*, const uint64_t*, size_t, uint64_t*) { return fail(B200_EINVAL, "pairing: not in this build variant"); }
 int fq12_mul_batch_host(const uint64_t*, const uint64_t*, size_t, uint64_t*) { return fail(B200_EINVAL, "fq12_mul: not in this build variant"); }
@@ -1196,6 +1423,14 @@ int groth16_verify_batch_host(const uint64_t*, size_t, const uint64_t*, const ui
                               const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*, size_t, const uint64_t*, int*,
                               uint64_t*) {
   return fail(B200_EINVAL, "groth16_verify_batch: not in this build variant");
+}
+int pinocchio_verify_host(const uint64_t*, size_t, const uint64_t*, const uint64_t*, const uint64_t*, const uint64_t*,
+                          const uint64_t*, size_t, int*, int*) {
+  return fail(B200_EINVAL, "pinocchio_verify: not in this build variant");
+}
+int pinocchio_verify_batch_host(const uint64_t*, size_t, const uint64_t*, const uint64_t*, size_t, const uint64_t*,
+                                const uint64_t*, const uint64_t*, size_t, const uint64_t*, int*, uint64_t*) {
+  return fail(B200_EINVAL, "pinocchio_verify_batch: not in this build variant");
 }
 #endif
 
@@ -1464,6 +1699,18 @@ int b200_groth16_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t al
                               const uint64_t* rho, int* ok, uint64_t stats[4]) {
   B200_API_BODY(groth16_verify_batch_host(ic, n_ic, alpha1, beta2, gamma2, delta2, nproofs, pi_a, pi_b, pi_c, public_signals,
                                           n_public, rho, ok, stats))
+}
+int b200_pinocchio_verify(const uint64_t* ic, size_t n_ic, const uint64_t vk_g1[24], const uint64_t vk_g2[120],
+                          const uint64_t proof_g1[84], const uint64_t pi_b[24], const uint64_t* public_signals,
+                          size_t n_public, int* ok, int* failed_check) {
+  B200_API_BODY(pinocchio_verify_host(ic, n_ic, vk_g1, vk_g2, proof_g1, pi_b, public_signals, n_public, ok, failed_check))
+}
+int b200_pinocchio_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t vk_g1[24], const uint64_t vk_g2[120],
+                                size_t nproofs, const uint64_t* proofs_g1, const uint64_t* pi_b,
+                                const uint64_t* public_signals, size_t n_public, const uint64_t* rho, int* ok,
+                                uint64_t stats[4]) {
+  B200_API_BODY(pinocchio_verify_batch_host(ic, n_ic, vk_g1, vk_g2, nproofs, proofs_g1, pi_b, public_signals, n_public, rho,
+                                            ok, stats))
 }
 int b200_g1_add_batch(const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out) { B200_API_BODY(group_op_host<Fq>(0, p, q, n, out)) }
 int b200_g1_double_batch(const uint64_t* p, size_t n, uint64_t* out) { B200_API_BODY(group_op_host<Fq>(1, p, nullptr, n, out)) }

@@ -9,7 +9,7 @@ import numpy as np
 from . import _lib
 from ._lib import check, ints_to_limbs, lib, ptr
 from .bn128 import R, _flatten_g1, _flatten_g2, _unflatten_g1, _unflatten_g2, reduce_scalar
-from .groth16 import KeyCache, _attr, _n_signals
+from .groth16 import KeyCache, _attr, _n_signals, _rand_rho
 
 _ORDER = ("PiA", "PiAp", "PiBp", "PiC", "PiCp", "PiH", "PiKp")
 
@@ -157,3 +157,42 @@ def VerifyProof(vk, proof, publicSignals, debug=False):
         if not ok:
             return False
     return True
+
+
+def _vk_limbs(vk):
+    """(IC, Vkb | G1Kbg, Vka | Vkc | Vkz | G2Kbg | G2Kg) in the layout of b200_pinocchio_verify."""
+    return (_flatten_g1(vk["IC"]), _flatten_g1([vk["Vkb"], vk["G1Kbg"]]),
+            _flatten_g2([vk["Vka"], vk["Vkc"], vk["Vkz"], vk["G2Kbg"], vk["G2Kg"]]))
+
+
+def VerifyProofBatch(vk, proofs, publicSignals, rho=None, stats=None):
+    """VerifyProof for every proofs[i] with publicSignals[i] under one vk, as one random linear combination on the GPU
+    (b200_pinocchio_verify_batch): the five checks of every proof raised to random powers and grouped by G2 point, one
+    Miller loop per proof and six for the key, one final exponentiation.  rho: per proof, five non-zero 128-bit scalars
+    (one per check), secret from whoever made the proofs; drawn here with ``secrets`` when None.  Returns a list of bools,
+    False wherever VerifyProof would return False or raise.  ``stats`` (a list) receives the library's counters: proofs in
+    the aggregated check, proofs verified one by one, aggregated checks run, Miller loops run."""
+    n = len(proofs)
+    if len(publicSignals) != n:
+        raise ValueError("VerifyProofBatch: one publicSignals list per proof")
+    if n == 0:
+        return []
+    npub = len(publicSignals[0])
+    if any(len(p) != npub for p in publicSignals):
+        raise ValueError("VerifyProofBatch: every proof needs the same number of public signals")
+    if rho is None:
+        rho = [[_rand_rho() for _ in range(5)] for _ in range(n)]
+    if len(rho) != n or any(len(r) != 5 or any(not 0 < int(x) < (1 << 128) for x in r) for r in rho):
+        raise ValueError("VerifyProofBatch: rho must be n lists of five non-zero 128-bit integers")
+    ic, vk1, vk2 = _vk_limbs(vk)
+    pg1 = _flatten_g1([p[k] for p in proofs for k in _ORDER])
+    pb = _flatten_g2([p["PiB"] for p in proofs])
+    pub = ints_to_limbs([reduce_scalar(x) for sig in publicSignals for x in sig]) if npub else np.zeros((1, 4), dtype=np.uint64)
+    rl = ints_to_limbs([int(x) for r in rho for x in r], 2)
+    ok = np.zeros(n, dtype=np.int32)
+    st = np.zeros(4, dtype=np.uint64)
+    check(lib().b200_pinocchio_verify_batch(ptr(ic), len(vk["IC"]), ptr(vk1), ptr(vk2), n, ptr(pg1), ptr(pb), ptr(pub), npub,
+                                            ptr(rl), ptr(ok), ptr(st)))
+    if stats is not None:
+        stats[:] = [int(x) for x in st]
+    return [bool(v == 1) for v in ok]

@@ -277,6 +277,33 @@ int b200_groth16_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t al
                               const uint64_t* pi_a, const uint64_t* pi_b, const uint64_t* pi_c,
                               const uint64_t* public_signals, size_t n_public, const uint64_t* rho,
                               int* ok, uint64_t stats[4]);
+/* snark.VerifyProof (snark.go:292-372) for one proof.  vk_g1 = Vkb | G1Kbg (2 x 12 u64), vk_g2 = Vka | Vkc | Vkz | G2Kbg |
+ * G2Kg (5 x 24 u64), proof_g1 = PiA, PiAp, PiBp, PiC, PiCp, PiH, PiKp (84 u64: the out_g1 order of b200_pinocchio_prove),
+ * pi_b = PiB.  *ok = 1 / 0; *failed_check (may be NULL) = 0, or 1..5 for the first of the reference's five checks that
+ * fails.  vkx = IC[0] + sum publicSignals[j] * IC[j+1], VkxA = vkx + PiA and VkxAC = VkxA + PiC use the reference's Add
+ * (Add(P, P) is infinity); a G1 point at infinity is paired as (0, 0), as the reference does.  The twelve pairings run
+ * concurrently.  Errors: null pointers or n_ic < n_public + 1 (B200_EINVAL); PiB or a vk G2 point at infinity (B200_EINVAL:
+ * the reference panics, bn128.go:238-241); otherwise a coordinate >= q or a public signal >= r (B200_ERANGE).  So when a
+ * G2 point at infinity and an out-of-range value occur together, B200_EINVAL wins.                                    */
+int b200_pinocchio_verify(const uint64_t* ic, size_t n_ic, const uint64_t vk_g1[24], const uint64_t vk_g2[120],
+                          const uint64_t proof_g1[84], const uint64_t pi_b[24], const uint64_t* public_signals,
+                          size_t n_public, int* ok, int* failed_check);
+/* Verify nproofs Pinocchio proofs under ONE verification key (b200_pinocchio_verify per proof).  proofs_g1: nproofs x 84
+ * u64, pi_b: nproofs x 24, public_signals: nproofs x n_public x 4, rho: nproofs x 5 x 2 u64 — the caller's secret,
+ * uniformly random, non-zero 128-bit batching scalars, one per check of each proof.  ok[i] = 1 / 0, or the negative code
+ * b200_pinocchio_verify would return for proof i alone.  stats (may be NULL) = { proofs in the aggregated check, proofs
+ * verified one by one, aggregated checks run, Miller loops run (12 per proof verified one by one) }.
+ * Check k of proof i is raised to rho_ik and the product of all of them is grouped by G2 point: one Miller loop per PiB_i
+ * (G1 side rho2 Vkb + rho4 VkxA_i + rho5 G1Kbg) and six for g2, Vka, Vkc, Vkz, G2Kbg, G2Kg — N + 6 Miller loops and one
+ * final exponentiation (a false accept has probability <= 2^-128 over rho).  A G1 point, VkxA or VkxAC at infinity, a G1
+ * point off the curve, PiB off the twist or outside G2 are verified one by one, as is every proof of a batch whose
+ * aggregated check fails.  Call-level errors, ok[] untouched: null pointers, nproofs == 0 or > 2^26, n_ic < n_public + 1,
+ * a rho == 0 (B200_EINVAL); a vk G2 point at infinity (B200_EINVAL) or else a vk coordinate >= q (B200_ERANGE); Vkb or
+ * G1Kbg at infinity or off the curve, an IC point off the curve, a vk G2 point off the twist or outside G2 (B200_EINVAL). */
+int b200_pinocchio_verify_batch(const uint64_t* ic, size_t n_ic, const uint64_t vk_g1[24], const uint64_t vk_g2[120],
+                                size_t nproofs, const uint64_t* proofs_g1, const uint64_t* pi_b,
+                                const uint64_t* public_signals, size_t n_public, const uint64_t* rho, int* ok,
+                                uint64_t stats[4]);
 
 /* ---- dense QAP API upstream of GenerateProofs (small n; the prove path consumes px) ---- */
 /* PolynomialField.R1CSToQAP (r1csqap/r1csqap.go:161-188).  a, b, c: n x m row-major R1CS matrices (coefficients
